@@ -26,6 +26,13 @@ Workload (BASELINE.json configs[1]): 15x15 separable Gaussian blur (sigma = 2.25
 `--impl reference` times the reference's own CPU implementation of the path instead (the C++ port under oracle/: the Zig
 reference cannot be built in this image) with all host threads, pinned (OMP_PROC_BIND=close) and first-touch placed, on the
 full 8192 x 8192 image.
+
+`--steps` sets the number of timed steps of every timed loop: the blur (weak and strong), e2e, each extra config and the
+`--impl reference` arm.  Only `cpu_baseline` keeps its best of 2 single-threaded passes (about 4 s each).
+
+`--dump-outputs DIR` writes DIR/gaussian_blur.npy: 256 rows of the image the headline's last timed step wrote (the weak or the strong
+partitioning, as `--scaling` picks at N > 1; every block's first and last 8 rows and a seeded choice of interior rows), and their row
+numbers in that image as DIR/gaussian_blur_rows.npy, so that two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -50,6 +57,7 @@ HALO = 7
 METRIC = "Mpixels/sec Gaussian-blur 8K RGBA f32"
 WORKLOAD = "gaussian_blur_15x15_sigma2.25_mirror_8192x8192_rgba_f32"
 ALGO_BYTES_PER_PX = 32  # read 16 B + write 16 B (SURVEY.md 8d)
+DUMP_ROWS = 256  # --dump-outputs: 256 x 8192 RGBA f32 = 32 MiB
 
 
 def measured_peak_gbs():
@@ -165,7 +173,7 @@ def run_reference(args, rank, world):
     taps = zo.gaussian_taps(SIGMA)
     for _ in range(max(1, min(args.warmup, 2))):
         cpu_reference_pass(zo, planes, outs, taps, threads)
-    steps = max(1, min(args.steps, 10))
+    steps = args.steps
     times = [cpu_reference_pass(zo, planes, outs, taps, threads) for _ in range(steps)]
     ms = float(np.mean(times)) * 1e3
     mpx = ROWS * COLS / 1e6 / (ms * 1e-3)
@@ -204,17 +212,41 @@ def time_steps(torch, dist, world, dev, fn, steps, warmup):
     return float(t.item()) / steps
 
 
+def dump_outputs(torch, dist, rank, world, block, out_dir):
+    """--dump-outputs: rows of the blurred image gathered on rank 0 in rank order, written as DIR/gaussian_blur.npy (DUMP_ROWS x COLS x 4
+    f32) and their row numbers in the whole image as DIR/gaussian_blur_rows.npy (f64, exact for integers).  The rows are every rank's
+    first and last 8 rows, which read the mirror border or a neighbour's rows, and a seeded choice of its interior rows."""
+    rows = block.shape[0]
+    inner = np.random.default_rng(0).choice(np.arange(8, rows - 8), max(DUMP_ROWS // world - 16, 0), replace=False)
+    idx = np.concatenate([np.arange(8), np.sort(inner), np.arange(rows - 8, rows)])
+    s = block[torch.from_numpy(idx).to(block.device)].contiguous()
+    if world > 1:
+        parts = [torch.empty_like(s) for _ in range(world)]
+        dist.all_gather(parts, s)
+        s = torch.cat(parts)
+    if rank == 0:
+        out_dir.mkdir(parents=True, exist_ok=True)
+        np.save(out_dir / "gaussian_blur.npy", s.cpu().numpy())
+        np.save(out_dir / "gaussian_blur_rows.npy", np.concatenate([r * rows + idx for r in range(world)]).astype(np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=200, help="timed steps of every timed loop (the blur, e2e, the extra configs, --impl reference) except cpu_baseline's best of 2")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="zignal_b200", choices=["zignal_b200", "reference"])
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"], help="which partitioning is the headline `value` at N > 1")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extra", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", type=Path,
+                    help="write a fixed sample of the output of the headline blur's last timed step (and its row numbers) to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "zignal_b200":
+        ap.error("--dump-outputs applies to --impl zignal_b200")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -262,6 +294,8 @@ def main():
     launches = L.zb_kernel_launch_count() - launches0
     kernel_name = L.zb_last_kernel().decode()
     comm.status()
+    if args.dump_outputs is not None and (world == 1 or args.scaling == "weak"):
+        dump_outputs(torch, dist, rank, world, dst.interior_tensor(), args.dump_outputs)
     # keep the GPU under the same load a little longer so the clock sampler sees it (every rank: the steps are collective)
     for _ in range(60):
         for _ in range(50):
@@ -318,8 +352,10 @@ def main():
     if world > 1:
         rows_s = ROWS // world
         s2, d2 = make_blocks(rows_s)
-        ms_strong = time_steps(torch, dist, world, dev, lambda: s2.conv_separable(d2, taps, taps, zb.BorderMode.MIRROR), max(args.steps, 50), args.warmup)
+        ms_strong = time_steps(torch, dist, world, dev, lambda: s2.conv_separable(d2, taps, taps, zb.BorderMode.MIRROR), args.steps, args.warmup)
         comm.status()
+        if args.dump_outputs is not None and args.scaling == "strong":
+            dump_outputs(torch, dist, rank, world, d2.interior_tensor(), args.dump_outputs)
         s2.free()
         d2.free()
         strong = {"scaling": "strong", "image": [ROWS, COLS], "rows_per_gpu": rows_s, "ms_per_step": ms_strong,
@@ -345,7 +381,7 @@ def main():
         np.ctypeslib.as_array(C.cast(hout, C.POINTER(C.c_float)), shape=(rows_e, COLS, 4))[:] = 0
         hi = zb.ZbImage(hin.value, rows_e, COLS, COLS)
         ho = zb.ZbImage(hout.value, rows_e, COLS, COLS)
-        esteps = max(2, min(args.steps, 5))
+        esteps = args.steps
         zb._ffi.check(L.zb_host_gaussian_blur(hi, ho, int(zb.PixFmt.RGBAF32), C.c_float(SIGMA)))  # warm-up
         if world > 1:
             dist.barrier()
@@ -378,7 +414,7 @@ def main():
                 g = torch.Generator(device=dev).manual_seed(3)
                 x = torch.randint(0, 256, (16384, 16384, 3), device=dev, dtype=torch.uint8, generator=g)
                 big, small = zb.Image.from_tensor(x), zb.Image.init(4096, 4096, zb.PixFmt.RGB8)
-                ms = time_steps(torch, dist, world, dev, lambda: big.resize(small, zb.Interpolation.BICUBIC), 50, 5)
+                ms = time_steps(torch, dist, world, dev, lambda: big.resize(small, zb.Interpolation.BICUBIC), args.steps, 5)
                 extra["c3_bicubic_16384_to_4096_rgb8"] = {"ms": ms, "algorithmic_bytes": 855638016, "frac_of_hbm_peak": 855638016 / (ms * 1e-3) / 1e9 / peak_x}
                 del x, big, small
                 # PCA (the "SVD step" config): Pca.fit's device core on n = 1,048,576 x dim 256 f32 -- column means + centring,
@@ -392,14 +428,14 @@ def main():
                 def gram():
                     return matrix.gemm_device(cen, cen, True, False, 1.0 / (X.shape[0] - 1), 0.0, None)
                 matrix.center_columns(X, mean, True, cen)
-                ms_gemm = time_steps(torch, dist, world, dev, gram, 20, 3)
+                ms_gemm = time_steps(torch, dist, world, dev, gram, args.steps, 3)
                 cov = gram()
-                ms_svd = time_steps(torch, dist, world, dev, lambda: matrix.svd_device(cov, True, False), 3, 1)
+                ms_svd = time_steps(torch, dist, world, dev, lambda: matrix.svd_device(cov, True, False), args.steps, 1)
 
                 def fit():
                     matrix.center_columns(X, mean, True, cen)
                     matrix.svd_device(gram(), True, False)
-                ms_fit = time_steps(torch, dist, world, dev, fit, 3, 1)
+                ms_fit = time_steps(torch, dist, world, dev, fit, args.steps, 1)
                 extra["pca_fit_1048576x256_f32"] = {"ms": ms_fit, "gemm_xtx_ms": ms_gemm, "svd_256x256_ms": ms_svd,
                                                     "gemm_tflops_fp32_accurate": 2.0 * X.shape[0] * 256 * 256 / (ms_gemm * 1e-3) / 1e12,
                                                     "kernel": L.zb_last_kernel().decode()}
@@ -423,7 +459,7 @@ def main():
                     zb._ffi.check(L.zb_rotate_into_batch(src0, 1080 * 1920, dst0, orows * ocols, per_call, int(zb.PixFmt.RGBA8), C.c_float(angle),
                                                          C.c_float(cs[0]), C.c_float(cs[1]), int(zb.Interpolation.BILINEAR), C.c_float(1 / 3),
                                                          C.c_float(1 / 3), int(zb.BorderMode.ZERO), torch.cuda.current_stream().cuda_stream))
-            ms = time_steps(torch, dist, world, dev, rot, 5, 2)
+            ms = time_steps(torch, dist, world, dev, rot, args.steps, 2)
             bytes_c4 = 26305936 * n_total
             extra["c4_rotate45_1024x1080p_rgba8"] = {"ms": ms, "frames": n_total, "frames_per_gpu": n_local, "algorithmic_bytes": bytes_c4,
                                                      "frac_of_hbm_peak": bytes_c4 / (ms * 1e-3) / 1e9 / (peak_x * world)}
@@ -438,7 +474,7 @@ def main():
             f = FeatureDistributionMatching(zb.PixFmt.RGB8)
             comm.fdm_set_target(f, zb.Image.from_tensor(t5))
             f.set_source(zb.Image.from_tensor(s5))
-            ms = time_steps(torch, dist, world, dev, lambda: comm.fdm_update(f), 50, 5)
+            ms = time_steps(torch, dist, world, dev, lambda: comm.fdm_update(f), args.steps, 5)
             f.status()
             comm.status()
             extra["c5_fdm_update_4096x4096_rgb8"] = {"ms": ms, "rows_per_gpu": rows5, "algorithmic_bytes": 150994944,

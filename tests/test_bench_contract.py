@@ -6,6 +6,9 @@ import subprocess
 import sys
 from pathlib import Path
 
+import numpy as np
+import pytest
+
 ROOT = Path(__file__).resolve().parents[1]
 
 
@@ -16,7 +19,7 @@ def _run(args, env=None, timeout=600):
 
 
 def test_reference_arm_prints_the_contract_line():
-    res = _run(["--impl", "reference", "--steps", "1", "--warmup", "1"])
+    res = _run(["--impl", "reference", "--steps", "12", "--warmup", "1"])
     assert res.returncode == 0, res.stderr[-2000:]
     lines = [ln for ln in res.stdout.splitlines() if ln.strip()]
     assert len(lines) == 1
@@ -26,6 +29,7 @@ def test_reference_arm_prints_the_contract_line():
     for key in ("value", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling", "vs_baseline", "dtype", "data", "config",
                 "cpu_baseline", "e2e"):
         assert key in line, key
+    assert line["steps"] == 12
     assert line["value"] > 0 and line["higher_is_better"] is True and line["vs_baseline"] is None and line["data"] == "synthetic"
     assert "workload" in line["config"] and "model" not in line["config"]
     cb = line["cpu_baseline"]
@@ -44,3 +48,36 @@ def test_product_arm_needs_cuda():
         return                                   # on a GPU box the driver runs the real thing
     res = _run(["--steps", "1", "--warmup", "3", "--no-e2e", "--no-cpu-baseline"], timeout=300)
     assert res.returncode != 0 and res.stdout.strip() == ""      # no JSON line from a CPU fallback: there is none
+
+
+@pytest.mark.gpu
+def test_dump_outputs_is_the_blur_of_the_last_step_whatever_the_step_count(tmp_path):
+    """--steps sets the timed launches, and --dump-outputs writes the same fixed sample of the blurred image on every run: rows of the
+    oracle's blur of the benchmark's seeded input."""
+    import torch
+
+    import oracle_lib as zo
+    from gpu_utils import rel_err
+    dumps = []
+    for steps in (1, 4):
+        d = tmp_path / f"steps{steps}"
+        res = _run(["--steps", str(steps), "--warmup", "3", "--no-e2e", "--no-cpu-baseline", "--no-extra", "--dump-outputs", str(d)])
+        assert res.returncode == 0, res.stderr[-2000:]
+        line = json.loads(res.stdout.strip().splitlines()[-1])
+        assert line["steps"] == steps and line["gpu_launches"] == steps
+        files = sorted(d.iterdir())
+        assert [f.name for f in files] == ["gaussian_blur.npy", "gaussian_blur_rows.npy"]
+        assert sum(f.stat().st_size for f in files) <= 64 << 20
+        dumps.append((np.load(files[0]), np.load(files[1])))
+    (a, rows), (b, rows_b) = dumps
+    assert a.shape == (256, 8192, 4) and a.dtype == np.float32 and rows.dtype == np.float64
+    assert np.array_equal(a, b) and np.array_equal(rows, rows_b)
+    rows = rows.astype(np.int64)
+    assert np.array_equal(rows[:8], np.arange(8)) and np.array_equal(rows[-8:], np.arange(8184, 8192)) and np.all(np.diff(rows) > 0)
+    # the benchmark's input (N = 1: rank 0's seed), blurred by the oracle in strips that hold every row a checked row reads
+    x = torch.rand(8192, 8192, 4, device="cuda", dtype=torch.float32, generator=torch.Generator(device="cuda").manual_seed(2))
+    taps = zo.gaussian_taps(2.25)
+    for lo, hi, check in [(0, 15, range(0, 8)), (8177, 8192, range(8184, 8192))] + [(r - 7, r + 8, [r]) for r in rows[8:-8:40]]:
+        want = zo.conv_separable(x[lo:hi].cpu().numpy(), taps, taps, "mirror")
+        for r in check:
+            assert rel_err(a[np.searchsorted(rows, r)], want[r - lo]) <= 1e-5, r
